@@ -380,12 +380,18 @@ def run_gpu(args):
     launches0 = eng.launch_count
     barrier()
     ev0.record()
-    run_pipelined_dev(args.steps)
+    timed_results = run_pipelined_dev(args.steps)
     ev1.record()
     barrier()
     ms_dev = ev0.elapsed_time(ev1) / args.steps
     launches = (eng.launch_count - launches0) // args.steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # what submit_dev's caller receives for the last timed epoch, copied now: later epochs reuse the pipeline slots
+        ok_last, head_last = timed_results[-1].wait()
+        dump = {"verdicts": ok_last.cpu().numpy().astype(np.float32),
+                "head_index": np.array([head_last], dtype=np.float64),
+                "aggregate_signatures": timed_results[-1].aggregate_signatures().cpu().numpy().astype(np.float32)}
 
     # ---- timed region 2: end to end through the public host API (pinned host buffers; H2D of every epoch's inputs and D2H of
     # its verdicts + head + aggregate signatures inside the region; copies of epoch k+1 overlap with the compute of epoch k)
@@ -611,6 +617,10 @@ def run_gpu(args):
                                     "sample": "%d of the 2048 committees of this epoch (512 members each), 1 per core, %.1f s wall: oracle bls.Aggregate + FastAggregateVerify" % (cores, wall),
                                     "aggregate_bytes_match_gpu": agg_match,
                                     "get_head_numpy_ms": cpu_head_ms, "get_head_matches_gpu": bool(hd_cpu == hd)}
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -634,7 +644,14 @@ def main():
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the per-config numbers of BASELINE.json configs 2 and 3")
     ap.add_argument("--probe-overlap", action="store_true",
                     help="also time bls.Aggregate and FastAggregateVerify running concurrently on two streams (diagnostic)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed epoch returned (rank 0: verdicts, head index, aggregate "
+                         "signatures) as DIR/<name>.npy in float32/float64; the seeded inputs make two builds comparable")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

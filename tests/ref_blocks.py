@@ -1,16 +1,10 @@
-"""Load the reference's own fenced ```python blocks from /root/reference/pos-evolution.md at test
-time (never copied into the repo) so they can be executed against the oracle's restated helpers.
-Only usable where /root/reference exists (the build container); the GPU box uses the golden
-fixtures generated from them (tests/golden/gen_golden.py)."""
+"""Load the reference's own fenced ```python blocks from pos-evolution.md (ethereum/pos-evolution; never
+copied into the repo) so they can be executed against the oracle's restated helpers.  Used by
+tests/golden/gen_golden.py, which records what they compute; the tests replay those vectors."""
 import __future__
-import os
 import re
 
-REF_MD = "/root/reference/pos-evolution.md"
-
-
-def available() -> bool:
-    return os.path.exists(REF_MD)
+REF_MD = None      # path of pos-evolution.md, set by the caller
 
 
 def fenced_blocks():

@@ -1,5 +1,6 @@
 """Deterministic synthetic inputs shared by the CPU and GPU tests (SURVEY.md section 8d).
 Uses the oracle to make keys/signatures -- test infrastructure only."""
+import copy
 import hashlib
 
 import numpy as np
@@ -105,6 +106,38 @@ def fork_tree(n_blocks: int, seed: int = 4):
     roots = np.frombuffer(b"".join(_h(i.to_bytes(8, "little")) for i in range(n_blocks)), dtype=np.uint8).reshape(n_blocks, 32).copy()
     leaf_viable = (rng.random(n_blocks) >= 0.05).astype(np.uint8)
     return parent, slot, roots, leaf_viable
+
+
+def small_store(spec, state, n_blocks=200, seed=3):
+    """An oracle Store over fork_tree(n_blocks, seed): non-viable leaves get a mismatching justified checkpoint, validators 3
+    and 17 equivocate, the proposer boost sits on the last block and ~90% of the validators hold a latest message."""
+    parent, slot, roots, leaf_viable = fork_tree(n_blocks, seed)
+    rb = [bytes(r) for r in roots]
+    just = S.Checkpoint(1, rb[0])
+    fin = S.Checkpoint(1, rb[0])
+    store = S.Store(time=0, genesis_time=0, justified_checkpoint=just, finalized_checkpoint=fin,
+                    best_justified_checkpoint=just, proposer_boost_root=rb[n_blocks - 1], equivocating_indices={3, 17})
+    has_child = set(int(p) for p in parent[1:])
+    for b in range(n_blocks):
+        store.blocks[rb[b]] = S.BeaconBlock(int(slot[b]), rb[parent[b]] if b else bytes(32))
+        bs = copy.copy(state)
+        if b not in has_child and not leaf_viable[b]:
+            bs.current_justified_checkpoint = S.Checkpoint(0, b"\x01" * 32)
+        else:
+            bs.current_justified_checkpoint = just
+        bs.finalized_checkpoint = fin
+        store.block_states[rb[b]] = bs
+    store.checkpoint_states[just] = state
+    rng = np.random.default_rng(seed)
+    n = len(state.validators)
+    for v in range(n):
+        if rng.random() < 0.9:
+            store.latest_messages[v] = S.LatestMessage(1, rb[int(n_blocks - 1 - min(n_blocks - 1, rng.geometric(0.05)))])
+    return store, parent, slot, roots, leaf_viable, rb
+
+
+# (epoch, voted block, attesting validators) of the update_latest_messages sequence the golden vectors record
+LMD_UPDATES = ((1, 10, [1, 2, 3, 40]), (2, 20, [2, 3, 17, 41, 63]), (1, 30, [2, 50]))
 
 
 def votes(n_validators: int, n_blocks: int, seed: int = 4):

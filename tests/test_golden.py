@@ -1,6 +1,5 @@
 """Golden vectors produced by executing the reference's own python blocks (tests/golden/gen_golden.py)
-replayed against (a) the oracle -- CPU, pins the oracle wherever /root/reference is absent -- and (b) the
-CUDA path through the pyspec-signature layer -- GPU."""
+replayed against (a) the oracle -- CPU -- and (b) the CUDA path through the pyspec-signature layer -- GPU."""
 import copy
 import json
 import os

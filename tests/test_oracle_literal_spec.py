@@ -1,51 +1,51 @@
-"""Differential tests: the reference's own fenced python blocks (executed from
-/root/reference/pos-evolution.md) vs the oracle's restatement vs the numpy array form.
-Skipped where /root/reference is absent (GPU box) -- there tests/test_golden.py replays the
-vectors these runs produced (tests/golden/gen_golden.py)."""
+"""Differential tests: what the reference's own fenced python blocks computed (pos-evolution.md, executed
+literally by tests/golden/gen_golden.py and stored in tests/golden/literal_spec.json) vs the oracle's
+restatement vs the numpy array form, on the same generated inputs."""
 import copy
-import hashlib
+import json
+import os
 
 import numpy as np
 import pytest
 
-import ref_blocks
 import scenarios
 from oracle import fast
 from oracle import spec as S
 
-pytestmark = pytest.mark.skipif(not ref_blocks.available(), reason="/root/reference not present")
+G = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "literal_spec.json")))
 
 
 @pytest.fixture(scope="module")
 def env():
-    import literal
     spec, state = scenarios.minimal_state(64, slot=9)
-    return spec, state, literal.namespace(spec)
+    assert [v.pubkey.hex() for v in state.validators] == G["pubkeys"]
+    return spec, state
 
 
 def test_shuffle_literal_vs_oracle_vs_numpy(env):
-    spec, _, ns = env
-    for n, tag in ((1, b"a"), (2, b"b"), (37, b"c"), (256, b"d"), (257, b"e"), (1000, b"f")):
-        seed = hashlib.sha256(tag).digest()
-        lit = [ns["compute_shuffled_index"](ns["uint64"](i), ns["uint64"](n), seed) for i in range(n)]
+    spec, _ = env
+    assert {s["n"] for s in G["shuffle"]} == {1, 2, 37, 256, 257, 1000}
+    for s in G["shuffle"]:
+        n, seed, lit = s["n"], bytes.fromhex(s["seed"]), s["perm"]
+        assert s["rounds"] == spec.p.SHUFFLE_ROUND_COUNT
         assert lit == [spec.compute_shuffled_index(i, n, seed) for i in range(n)]
         assert lit == fast.shuffle_permutation(n, seed, spec.p.SHUFFLE_ROUND_COUNT).tolist()
         assert sorted(lit) == list(range(n))
 
 
 def test_committees_literal_vs_numpy(env):
-    spec, state, ns = env
+    spec, state = env
     epoch = 1
-    cps = ns["get_committee_count_per_slot"](state, epoch)
+    cps = G["committee_count_per_slot"][str(epoch)]
     assert cps == 2 == spec.get_committee_count_per_slot(state, epoch)
-    seed = ns["get_seed"](state, epoch, S.DOMAIN_BEACON_ATTESTER)
-    assert seed == spec.get_seed(state, epoch, S.DOMAIN_BEACON_ATTESTER)
+    seed = spec.get_seed(state, epoch, S.DOMAIN_BEACON_ATTESTER)
+    assert seed.hex() == G["attester_seed"][str(epoch)]
     active = np.array(spec.get_active_validator_indices(state, epoch), dtype=np.uint32)
     members, off = fast.committees_for_epoch(active, seed, spec.p.SHUFFLE_ROUND_COUNT, cps, spec.p.SLOTS_PER_EPOCH)
     seen = []
     for s in range(spec.p.SLOTS_PER_EPOCH):
         for c in range(cps):
-            lit = ns["get_beacon_committee"](state, epoch * spec.p.SLOTS_PER_EPOCH + s, c)
+            lit = G["committees"]["%d/%d" % (epoch * spec.p.SLOTS_PER_EPOCH + s, c)]
             k = s * cps + c
             assert lit == members[off[k]:off[k + 1]].tolist() == spec.get_beacon_committee(state, 8 + s, c)
             assert len(lit) == 4
@@ -63,7 +63,7 @@ def _run(fn, state, att):
 
 
 def test_process_attestation_literal_vs_oracle(env):
-    spec, state, ns = env
+    spec, state = env
     cases = [
         scenarios.make_attestation(spec, state, 8, 0),
         scenarios.make_attestation(spec, state, 8, 1, bits=[True, False, True, False]),
@@ -78,55 +78,35 @@ def test_process_attestation_literal_vs_oracle(env):
     bad_idx.data = S.AttestationData(8, 2, bad_idx.data.beacon_block_root, bad_idx.data.source, bad_idx.data.target)
     cases.append(bad_idx)                                                                 # index >= committee count
     expect = ["ok", "ok", "ok", "assert", "assert", "assert", "assert", "assert", "assert"]
-    for att, exp in zip(cases, expect):
-        r_lit, st_lit = _run(ns["process_attestation"], state, att)
+    assert len(G["process_attestation"]) == len(cases)
+    for att, exp, lit in zip(cases, expect, G["process_attestation"]):
+        assert lit["attestation"]["signature"] == att.signature.hex() and lit["attestation"]["index"] == att.data.index
+        assert lit["attestation"]["bits"] == [bool(b) for b in att.aggregation_bits]
         r_or, st_or = _run(spec.process_attestation, state, att)
-        assert r_lit == r_or == exp
+        assert lit["result"] == r_or == exp
         if exp == "ok":
-            assert st_lit.current_epoch_participation == st_or.current_epoch_participation
-            assert st_lit.previous_epoch_participation == st_or.previous_epoch_participation
-            assert st_lit.balances == st_or.balances
-            assert st_lit.balances != state.balances
+            assert lit["current_epoch_participation"] == st_or.current_epoch_participation
+            assert lit["previous_epoch_participation"] == st_or.previous_epoch_participation
+            assert lit["balances"] == st_or.balances
+            assert lit["balances"] != state.balances
     # double inclusion: flags already set -> no second reward
+    twice = G["process_attestation_twice"]
+    assert twice["balances_after_first"] == G["process_attestation"][0]["balances"]
+    assert twice["balances_after_second"] == twice["balances_after_first"]
     st = copy.deepcopy(state)
-    ns["process_attestation"](st, cases[0])
-    b1 = list(st.balances)
-    ns["process_attestation"](st, cases[0])
-    assert st.balances == b1
-
-
-def _small_store(spec, state, n_blocks=200, seed=3):
-    parent, slot, roots, leaf_viable = scenarios.fork_tree(n_blocks, seed)
-    rb = [bytes(r) for r in roots]
-    just = S.Checkpoint(1, rb[0])
-    fin = S.Checkpoint(1, rb[0])
-    store = S.Store(time=0, genesis_time=0, justified_checkpoint=just, finalized_checkpoint=fin,
-                    best_justified_checkpoint=just, proposer_boost_root=rb[n_blocks - 1], equivocating_indices={3, 17})
-    has_child = set(int(p) for p in parent[1:])
-    for b in range(n_blocks):
-        store.blocks[rb[b]] = S.BeaconBlock(int(slot[b]), rb[parent[b]] if b else bytes(32))
-        bs = copy.copy(state)
-        if b not in has_child and not leaf_viable[b]:
-            bs.current_justified_checkpoint = S.Checkpoint(0, b"\x01" * 32)
-        else:
-            bs.current_justified_checkpoint = just
-        bs.finalized_checkpoint = fin
-        store.block_states[rb[b]] = bs
-    store.checkpoint_states[just] = state
-    rng = np.random.default_rng(seed)
-    n = len(state.validators)
-    for v in range(n):
-        if rng.random() < 0.9:
-            store.latest_messages[v] = S.LatestMessage(1, rb[int(n_blocks - 1 - min(n_blocks - 1, rng.geometric(0.05)))])
-    return store, parent, slot, roots, leaf_viable, rb
+    spec.process_attestation(st, cases[0])
+    assert st.balances == twice["balances_after_first"]
+    spec.process_attestation(st, cases[0])
+    assert st.balances == twice["balances_after_second"]
 
 
 def test_get_head_literal_vs_oracle_vs_numpy(env):
-    spec, state, ns = env
+    spec, state = env
     state = copy.deepcopy(state)
     state.validators[5].exit_epoch = 0          # inactive validator is not counted
-    store, parent, slot, roots, leaf_viable, rb = _small_store(spec, state)
-    head_lit = ns["get_head"](store)
+    store, parent, slot, roots, leaf_viable, rb = scenarios.small_store(spec, state)
+    assert {str(v): [m.epoch, m.root.hex()] for v, m in store.latest_messages.items()} == G["get_head"]["latest_messages"]
+    head_lit = bytes.fromhex(G["get_head"]["head"])
     assert head_lit == spec.get_head(store)
     n = len(state.validators)
     idx_of = {r: i for i, r in enumerate(rb)}
@@ -148,8 +128,9 @@ def test_get_head_literal_vs_oracle_vs_numpy(env):
 
 
 def test_update_latest_messages_literal_vs_numpy(env):
-    spec, state, ns = env
-    store, parent, slot, roots, leaf_viable, rb = _small_store(spec, state, n_blocks=50)
+    spec, state = env
+    g = G["update_latest_messages"]
+    store, parent, slot, roots, leaf_viable, rb = scenarios.small_store(spec, state, n_blocks=g["n_blocks"], seed=g["tree_seed"])
     n = len(state.validators)
     idx_of = {r: i for i, r in enumerate(rb)}
     msg_epoch = np.zeros(n, dtype=np.uint64)
@@ -159,36 +140,34 @@ def test_update_latest_messages_literal_vs_numpy(env):
         msg_epoch[v], msg_block[v], has_msg[v] = lm.epoch, idx_of[lm.root], 1
     equiv = np.zeros(n, dtype=np.uint8)
     equiv[list(store.equivocating_indices)] = 1
-    for epoch, blk, idxs in ((1, 10, [1, 2, 3, 40]), (2, 20, [2, 3, 17, 41, 63]), (1, 30, [2, 50])):
-        att = S.Attestation([], S.AttestationData(0, 0, rb[blk], S.Checkpoint(), S.Checkpoint(epoch, rb[0])), b"")
-        ns["update_latest_messages"](store, idxs, att)
+    for epoch, blk, idxs in scenarios.LMD_UPDATES:
         fast.lmd_update(msg_epoch, msg_block, has_msg, equiv, idxs, epoch, blk)
+    lit = {int(v): tuple(m) for v, m in g["latest_messages"].items()}
     for v in range(n):
         if has_msg[v]:
-            assert store.latest_messages[v] == S.LatestMessage(int(msg_epoch[v]), rb[msg_block[v]])
+            assert lit[v] == (int(msg_epoch[v]), int(msg_block[v]))
         else:
-            assert v not in store.latest_messages
+            assert v not in lit
 
 
 def test_ffg_literal_vs_oracle(env):
-    """process_justification_and_finalization / weigh_justification_and_finalization: the reference's own text (ref :793-852)
-    against the oracle's restatement on 80 generated end-of-epoch states; every branch must have fired."""
-    import copy
-    spec, state0, ns = env[0], env[1], env[2]
+    """process_justification_and_finalization / weigh_justification_and_finalization: what the reference's own text (ref :793-852)
+    computed against the oracle's restatement on 80 generated end-of-epoch states; every branch must have fired."""
+    spec, state0 = env
+    assert [c["seed"] for c in G["ffg"]] == list(range(80))
     seen = set()
-    for seed in range(80):
-        st_ref = scenarios.ffg_case(copy.deepcopy(state0), seed)
-        st_or = copy.deepcopy(st_ref)
-        before = (st_ref.current_justified_checkpoint, st_ref.finalized_checkpoint)
-        ns["process_justification_and_finalization"](st_ref)
+    for case in G["ffg"]:
+        seed = case["seed"]
+        st_or = scenarios.ffg_case(copy.deepcopy(state0), seed)
+        before = (scenarios.ffg_outcome(st_or)["current_justified"], scenarios.ffg_outcome(st_or)["finalized"])
         spec.process_justification_and_finalization(st_or)
-        got, want = scenarios.ffg_outcome(st_or), scenarios.ffg_outcome(st_ref)
+        got, want = scenarios.ffg_outcome(st_or), {k: v for k, v in case.items() if k != "seed"}
         assert got == want, seed
-        seen.add(("justified_changed", st_ref.current_justified_checkpoint != before[0]))
-        seen.add(("finalized_changed", st_ref.finalized_checkpoint != before[1]))
+        seen.add(("justified_changed", want["current_justified"] != before[0]))
+        seen.add(("finalized_changed", want["finalized"] != before[1]))
         seen.add(("bits", tuple(want["justification_bits"][:2])))
-        if st_ref.finalized_checkpoint != before[1]:
-            seen.add(("finalized_distance", spec.get_current_epoch(st_ref) - st_ref.finalized_checkpoint.epoch))
+        if want["finalized"] != before[1]:
+            seen.add(("finalized_distance", spec.get_current_epoch(st_or) - want["finalized"][0]))
     assert {("justified_changed", True), ("justified_changed", False), ("finalized_changed", True), ("finalized_changed", False)} <= seen
     assert {("bits", (0, 0)), ("bits", (0, 1)), ("bits", (1, 0)), ("bits", (1, 1))} <= seen
     assert {("finalized_distance", 1), ("finalized_distance", 2), ("finalized_distance", 3)} <= seen
